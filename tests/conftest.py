@@ -43,11 +43,11 @@ def real_gpu():
 
 @pytest.fixture(scope="session")
 def ref():
-    """The unmodified reference runtime (oracle/_ref); skipped if not built."""
+    """The unmodified reference runtime (oracle/_ref), or where it is not built
+    the answers it gave, recorded under tests/golden/ref_results."""
     import oracle.ref as r
     if not r.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    r.lib()
+        pytest.skip("oracle/_ref not built and no recorded reference answers")
     return r
 
 

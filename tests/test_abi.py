@@ -114,18 +114,10 @@ def test_serialize_roundtrip_and_errors(hs, ref):
 
 def test_reference_accepts_our_database_container(hs, ref):
     """The reference's own hs_deserialize/hs_database_info read our container."""
-    R = ref.lib()
     db = hs.compile_lit_multi([b"needle"])
-    blob = db.serialize()
-    out = C.c_void_p()
-    R.hs_deserialize_database.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_void_p)]
-    assert R.hs_deserialize_database(blob, len(blob), C.byref(out)) == 0
-    info = C.c_char_p()
-    R.hs_database_info.argtypes = [C.c_void_p, C.POINTER(C.c_char_p)]
-    assert R.hs_database_info(out, C.byref(info)) == 0
-    assert b"5.4.2" in info.value and b"BLOCK" in info.value
-    data = b"xxneedlexx"
-    r = ref.scan_sorted(out.value, data, [0], [len(data)])
+    rc, info, r = ref.read_container(db.serialize(), b"xxneedlexx")
+    assert rc == 0
+    assert "5.4.2" in info and "BLOCK" in info
     assert [(int(x["id"]), int(x["to"])) for x in r] == [(0, 8)]
 
 

@@ -43,9 +43,10 @@ def test_emitted_engines_run_on_the_reference(hs, ref, kind, nlits, alphabet, lo
     lits, flags, ids, data, off, ln = _lit_case(nlits, nlits, alphabet, lo, hi, 0.0 if kind == "sheng" else 0.2)
     eng = hs.dfa_from_literals(lits, [f & 1 for f in flags], ids, kind=KINDS[kind], sherman=sherman)
     assert eng[8] in (6, 7, 17)                                   # NFA.type
-    got = ref.nfa_exec_blocks(eng, data, off, ln)
+    want = _definition(lits, flags, ids, data, off, ln)
+    got = ref.nfa_exec_blocks(eng, data, off, ln, like=want)
     # the reference fires one callback per report of the accept state's list: a set per (block, to)
-    assert _triples(got) == _definition(lits, flags, ids, data, off, ln)
+    assert _triples(got) == want
 
 
 def _random_table(seed, nstates, nreports=5, dead_frac=0.1):
@@ -98,8 +99,9 @@ def test_random_tables_reference_equals_definition(hs, ref, kind, nstates, sherm
     lens = [0, 1, 5, 16, 17, 200, 1024]
     data, off, ln = synth.ragged_corpus(lens, None, seed=nstates, plant_per_kb=0)
     data = rng.integers(0, 256, size=data.size, dtype=np.uint8)
-    got = ref.nfa_exec_blocks(eng, data, off, ln)
-    assert _triples(got) == _walk(nxt, reports, eod, 1, data, off, ln)
+    want = _walk(nxt, reports, eod, 1, data, off, ln)
+    got = ref.nfa_exec_blocks(eng, data, off, ln, like=want)
+    assert _triples(got) == want
 
 
 def test_builder_refuses_what_does_not_fit(hs):
@@ -121,7 +123,7 @@ def test_device_engines_equal_reference_literals(hs, ref, kind, nlits, alphabet,
     eng = hs.dfa_from_literals(lits, [f & 1 for f in flags], ids, kind=KINDS[kind], sherman=sherman)
     corpus = hs.Corpus.upload(data, off, ln)
     got, ms = hs.nfa_scan_corpus(eng, corpus)
-    want = ref.nfa_exec_blocks(eng, data, off, ln)
+    want = ref.nfa_exec_blocks(eng, data, off, ln, like=got)
     assert _triples(got) == _triples(want)
     assert len(want) > 20
     corpus.free()
@@ -141,7 +143,7 @@ def test_device_engines_equal_reference_random_tables(hs, ref, kind, nstates, sh
         nxt, reports, eod = _random_table(3 * nstates + sherman + 1000 * k, nstates)
         eng = hs.dfa_from_table(nxt, 1, 1, reports, eod, kind=KINDS[kind], sherman=sherman)
         got, ms = hs.nfa_scan_corpus(eng, corpus, cap=64)        # forces the grow-and-retry path
-        want = ref.nfa_exec_blocks(eng, data, off, ln)
+        want = ref.nfa_exec_blocks(eng, data, off, ln, like=got)
         assert _triples(got) == _triples(want)
         busy += len(want) > 100
     assert busy >= 2
@@ -157,7 +159,7 @@ def test_device_dfa_uniform_blocks_and_big_table(hs, ref):
     data, off, ln, _ = synth.block_corpus(512, 1024, lits, plant_per_kb=1.0, seed=10)
     corpus = hs.Corpus.upload(data, off, ln)
     got, ms = hs.nfa_scan_corpus(eng, corpus)
-    want = ref.nfa_exec_blocks(eng, data, off, ln)
+    want = ref.nfa_exec_blocks(eng, data, off, ln, like=got)
     assert _triples(got) == _triples(want) and len(want) > 300
     corpus.free()
 

@@ -53,17 +53,7 @@ def find(hs, typ, params, data):
 
 
 def ref_find(ref, typ, params, data):
-    R = ref.lib()
-    buf = np.zeros(len(data) + 192, dtype=np.uint8)
-    buf[64:64 + len(data)] = np.frombuffer(bytes(data), dtype=np.uint8)
-    p = buf.ctypes.data + 64
-    if typ == SHUFTI:
-        return R.ref_shufti(params[:16], params[16:], p, len(data))
-    if typ == TRUFFLE:
-        return R.ref_truffle(params[:16], params[16:], p, len(data))
-    if typ in (VERM, VERM_NC):
-        return R.ref_vermicelli(params[0], typ == VERM_NC, p, len(data))
-    return R.ref_dvermicelli(params[0], params[1], typ == DVERM_NC, p, len(data))
+    return ref.accel_find(typ, params, data)
 
 
 def test_shufti_exec_match1_kat(hs, ref):

@@ -33,11 +33,12 @@ def test_literal_nfas_run_on_the_reference(hs, ref, i):
     lits, cl, ids, data, off, ln = _lit_case(i)
     eng = hs.limex32_from_literals(lits, cl, ids)
     assert eng[8] == (0 if sum(map(len, lits)) < 32 else 1)            # NFA.type = LIMEX_NFA_32 / _64
-    got = _triples(ref.nfa_exec_blocks(eng, data, off, ln))
+    walk = model.walk_blocks(eng, data, off, ln)
+    got = _triples(ref.nfa_exec_blocks(eng, data, off, ln, like=walk))
     want = brute.scan_blocks(lits, cl, ids, data, off, ln)
     # one callback per accepting STATE: two literals with one report id ending together fire it twice
     assert sorted(set(got)) == sorted({(int(r["id"]), int(r["block"]), int(r["to"])) for r in want})
-    assert got == sorted(model.walk_blocks(eng, data, off, ln))
+    assert got == sorted(walk)
     assert len(got) > 20
 
 
@@ -92,8 +93,9 @@ def test_random_nfas_reference_equals_restatement(hs, ref, seed, wide):
     eng = _emit(hs, _random_nfa(seed, wide))
     assert eng[8] == (1 if wide else 0)
     data, off, ln = _random_corpus(100 + seed)
-    got = _triples(ref.nfa_exec_blocks(eng, data, off, ln))
-    assert got == sorted(model.walk_blocks(eng, data, off, ln))
+    walk = model.walk_blocks(eng, data, off, ln)
+    got = _triples(ref.nfa_exec_blocks(eng, data, off, ln, like=walk))
+    assert got == sorted(walk)
 
 
 def _random_wide_nfa(seed, n):
@@ -139,8 +141,9 @@ def test_random_wide_nfas_reference_equals_restatement(hs, ref, n, kind):
         eng = hs.limex_from_spec_wide(reach, init, init, succ, reports, eod, sqm, sk)
         assert eng[8] == kind                                         # LIMEX_NFA_128 / _256 / _512
         data, off, ln = _random_corpus(300 + seed)
-        got = _triples(ref.nfa_exec_blocks(eng, data, off, ln))
-        assert got == sorted(model.walk_blocks(eng, data, off, ln))
+        walk = model.walk_blocks(eng, data, off, ln)
+        got = _triples(ref.nfa_exec_blocks(eng, data, off, ln, like=walk))
+        assert got == sorted(walk)
         assert len(got) > 50
 
 
@@ -163,7 +166,7 @@ def test_device_limex_equals_reference_literals(hs, ref, i):
     eng = hs.limex32_from_literals(lits, cl, ids)
     corpus = hs.Corpus.upload(data, off, ln)
     got, ms = hs.nfa_scan_corpus(eng, corpus)
-    assert _triples(got) == _triples(ref.nfa_exec_blocks(eng, data, off, ln))
+    assert _triples(got) == _triples(ref.nfa_exec_blocks(eng, data, off, ln, like=got))
     corpus.free()
 
 
@@ -175,7 +178,7 @@ def test_device_limex_equals_reference_random(hs, ref, seed, wide):
     data, off, ln = _random_corpus(200 + seed)
     corpus = hs.Corpus.upload(data, off, ln)
     got, ms = hs.nfa_scan_corpus(eng, corpus, cap=64)                 # forces the grow-and-retry path
-    want = ref.nfa_exec_blocks(eng, data, off, ln)
+    want = ref.nfa_exec_blocks(eng, data, off, ln, like=got)
     assert _triples(got) == _triples(want)
     corpus.free()
 
@@ -190,7 +193,7 @@ def test_device_wide_limex_equals_reference_random(hs, ref, n, kind):
         data, off, ln = _random_corpus(300 + seed)
         corpus = hs.Corpus.upload(data, off, ln)
         got, ms = hs.nfa_scan_corpus(eng, corpus, cap=64)
-        assert _triples(got) == _triples(ref.nfa_exec_blocks(eng, data, off, ln))
+        assert _triples(got) == _triples(ref.nfa_exec_blocks(eng, data, off, ln, like=got))
         corpus.free()
 
 
@@ -203,7 +206,7 @@ def test_device_wide_limex_literals(hs, ref, reps, kind):
     data, off, ln, _ = synth.block_corpus(512, 1024, lits, plant_per_kb=2.0, seed=12)
     corpus = hs.Corpus.upload(data, off, ln)
     got, ms = hs.nfa_scan_corpus(eng, corpus)
-    want = ref.nfa_exec_blocks(eng, data, off, ln)
+    want = ref.nfa_exec_blocks(eng, data, off, ln, like=got)
     assert _triples(got) == _triples(want) and len(want) > 300
     corpus.free()
 
@@ -215,7 +218,7 @@ def test_device_limex_uniform_blocks(hs, ref):
     data, off, ln, _ = synth.block_corpus(2048, 1024, lits, plant_per_kb=2.0, seed=12)
     corpus = hs.Corpus.upload(data, off, ln)
     got, ms = hs.nfa_scan_corpus(eng, corpus)
-    want = ref.nfa_exec_blocks(eng, data, off, ln)
+    want = ref.nfa_exec_blocks(eng, data, off, ln, like=got)
     assert _triples(got) == _triples(want) and len(want) > 1000
     corpus.free()
 

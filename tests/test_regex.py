@@ -209,8 +209,8 @@ def test_device_scans_compiled_expressions(hs, ref, pi):
     a = np.frombuffer(ALPHA, dtype=np.uint8)
     data, off, ln = synth.ragged_corpus(lens, None, seed=pi, plant_per_kb=0)
     data = a[rng.integers(0, a.size, size=data.size)].astype(np.uint8)
-    want = ref.scan_sorted(db.ptr, data, off, ln)
     got = np.sort(hs.scan_blocks(db, data, off, ln, scratch), order=["block", "to", "id"])
+    want = ref.scan_sorted(db.ptr, data, off, ln, like=got)
     assert np.array_equal(got, want)
     b = 8
     buf = data[int(off[b]):int(off[b]) + int(ln[b])].tobytes()
@@ -224,9 +224,9 @@ def test_device_expression_set_with_report_rules(hs, ref):
     pats = [rb"ab+", rb"b+c", rb"[xy]z", rb"a.c", rb"\d{2,}"]
     db = hs.compile_multi(pats, [0, 0, SINGLE, 0, CASELESS], [1, 1, 2, 3, 4])
     data, off, ln, _ = synth.block_corpus(512, 512, [b"abbbc", b"xz", b"a1c22"], plant_per_kb=8.0, seed=3)
-    want = ref.scan_sorted(db.ptr, data, off, ln)
     scratch = hs.Scratch(db)
     got = np.sort(hs.scan_blocks(db, data, off, ln, scratch), order=["block", "to", "id"])
+    want = ref.scan_sorted(db.ptr, data, off, ln, like=got)
     assert np.array_equal(got, want) and want.size > 500
     scratch.free()
 

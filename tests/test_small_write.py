@@ -48,7 +48,7 @@ def test_reference_small_write_path_on_our_engines(hs, ref, nl, alphabet, lo, hi
     lens = list(range(0, 70)) * 3 + [70, 71, 100, 5000]           # < 70: small-write DFA; >= 70: rose
     data, o, l = synth.ragged_corpus(lens, lits, seed=nl, plant_per_kb=300, alphabet=alphabet + b"AB")
     want = brute.scan_blocks(lits, flags, ids, data, o, l)
-    got = ref.scan_sorted(db.ptr, data, o, l)
+    got = ref.scan_sorted(db.ptr, data, o, l, like=want)
     assert np.array_equal(got, want)
     assert want.size > 50
 
@@ -69,7 +69,7 @@ def test_device_equals_reference_on_short_buffers(hs, ref, nl, alphabet, lo, hi,
     data, o, l = synth.ragged_corpus(lens, lits, seed=nl, plant_per_kb=300, alphabet=alphabet + b"AB")
     scratch = hs.Scratch(db)
     got = np.sort(hs.scan_blocks(db, data, o, l, scratch), order=["block", "to", "id"])
-    assert np.array_equal(got, ref.scan_sorted(db.ptr, data, o, l))
+    assert np.array_equal(got, ref.scan_sorted(db.ptr, data, o, l, like=got))
     # and the engine itself on the device: the DFA's reports are report-program offsets
     bc = db.serialize()[32:]
     off = _small_write(db)[0]
@@ -77,7 +77,7 @@ def test_device_equals_reference_on_short_buffers(hs, ref, nl, alphabet, lo, hi,
     eng = bytes(bc[off + 64:off + size])
     corpus = hs.Corpus.upload(data, o, l)
     recs, ms = hs.nfa_scan_corpus(eng, corpus)
-    want = ref.nfa_exec_blocks(eng, data, o, l)
+    want = ref.nfa_exec_blocks(eng, data, o, l, like=recs)
     assert np.array_equal(np.sort(recs, order=["block", "to", "id"]), want) and want.size > 50
     corpus.free()
     scratch.free()

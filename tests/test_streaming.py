@@ -59,10 +59,7 @@ def test_stream_compile_rules(hs, ref):
     sz = ctypes.c_size_t()
     assert hs.lib().hs_stream_size(db.ptr, ctypes.byref(sz)) == 0
     assert sz.value == 16 + 1 + 1 + 7            # struct hs_stream + status + groups + history (src/runtime.c:1058)
-    rsz = ctypes.c_size_t()
-    R = ref.lib()
-    R.hs_stream_size.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_size_t)]
-    assert R.hs_stream_size(db.ptr, ctypes.byref(rsz)) == 0 and rsz.value == sz.value
+    assert ref.stream_size(db.ptr) == (0, sz.value)
     info = ctypes.c_void_p()
     assert hs.lib().hs_database_info(db.ptr, ctypes.byref(info)) == 0
     assert b"Mode: STREAM" in ctypes.string_at(info)
