@@ -7,6 +7,7 @@ fallback for the scan path.
 """
 import ctypes as C
 import os
+import struct
 
 import numpy as np
 
@@ -188,6 +189,27 @@ class Database:
         out = C.c_void_p()
         _check(lib().hs_deserialize_database(b, len(b), C.byref(out)))
         return Database(out)
+
+    def engines(self):
+        """The engines of an outfix database, one per queue in queue order: [(model, states)], model one of
+        ENGINE_MODELS' values, states the engine's NFA.nPositions.  [] for a database without engines."""
+        bc = self.serialize()[32:]  # the bytecode follows the 32-byte serialization header
+        n, info_at = struct.unpack_from("<I", bc, _ROSE_QUEUE_COUNT)[0], struct.unpack_from("<I", bc, _ROSE_NFA_INFO)[0]
+        if not info_at:
+            return []
+        out = []
+        for q in range(n):
+            nfa = struct.unpack_from("<I", bc, info_at + q * _NFA_INFO_SIZE)[0]
+            out.append((ENGINE_MODELS.get(bc[nfa + _NFA_TYPE], "type %d" % bc[nfa + _NFA_TYPE]),
+                        struct.unpack_from("<I", bc, nfa + _NFA_POSITIONS)[0]))
+        return out
+
+
+# NFA.type (src/nfa/nfa_internal.h:53-78) of the engines this library builds
+ENGINE_MODELS = {0: "LimEx-32", 1: "LimEx-64", 2: "LimEx-128", 3: "LimEx-256", 5: "LimEx-512", 6: "McClellan-8",
+                 7: "McClellan-16", 17: "Sheng"}
+# byte offsets of RoseEngine.queueCount, RoseEngine.nfaInfoOffset, sizeof(NfaInfo), NFA.type, NFA.nPositions
+_ROSE_QUEUE_COUNT, _ROSE_NFA_INFO, _NFA_INFO_SIZE, _NFA_TYPE, _NFA_POSITIONS = 156, 236, 20, 8, 20
 
 
 def _raise_compile(rc, err):

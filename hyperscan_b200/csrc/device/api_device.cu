@@ -130,8 +130,10 @@ struct DevImage {
     u32 bitmapBytes = 0, bitmapShift = 0, keyBytes = 0;
     u32 pairBytes = 0, bitmapHoles = 0, bitmapBits = 0; /* FK_PAIR32 layout (kernels.h) */
     u32 bucketFold = 0;
-    u32 nfaOffset = 0, nfaLength = 0;   /* FK_OUTFIX: the sole engine (bytecode offset, NFA.length) */
-    DfaParams nfaParams;                /* ... and what launchDfa needs to know about it */
+    /* FK_OUTFIX: the engines (one per queue), grouped by model, and one launch per model: `engines` of each
+     * launch points into d_engines */
+    DfaEngine *d_engines = nullptr;
+    std::vector<DfaParams> engineLaunches;
     /* FK_OUTFIX: report program offset -> its (onmatch, offset_adjust) list, filled as programs are met */
     mutable std::unordered_map<u32, std::vector<ProgReport>> progReports;
     double pairRate = 0;     /* FK_PAIR32: modelled first-stage candidates per byte (printable ASCII) */
@@ -606,6 +608,7 @@ void freeImage(DevImage *im) {
         return;
     }
     cudaFree(im->d_bc);
+    cudaFree(im->d_engines);
     cudaFree(im->d_table);
     cudaFree(im->d_bitmap);
     cudaFree(im->d_bitmap2);
@@ -622,8 +625,8 @@ hs_error_t buildImage(const hs_database_t *db, DevImage **out) {
     const bool soleOutfix = r->runtimeImpl == RUNTIME_SINGLE_OUTFIX && r->mode == MODE_BLOCK && r->queueCount == 1 &&
                             r->outfixBeginQueue == 0 && r->outfixEndQueue == 1 && r->nfaInfoOffset &&
                             !r->amatcherOffset && !r->ematcherOffset && !r->fmatcherOffset && !r->hasSom;
-    if (!soleOutfix && (r->runtimeImpl != RUNTIME_PURE_LITERAL || !r->fmatcherOffset)) {
-        /* FULL_ROSE databases need the full rose interpreter and the catch-up machinery
+    if (!soleOutfix && !outfixesOnly(r, h->length) && (r->runtimeImpl != RUNTIME_PURE_LITERAL || !r->fmatcherOffset)) {
+        /* other FULL_ROSE databases need the full rose interpreter and the catch-up machinery
          * (SURVEY.md section 8f rank 1): not in this build */
         return HS_ARCH_ERROR;
     }
@@ -645,45 +648,80 @@ hs_error_t buildImage(const hs_database_t *db, DevImage **out) {
     im->groups = r->initialGroups & r->floating_group_mask;
     im->minWidth = r->minWidth;
     im->hasDedupe = r->dkeyCount != 0;
-    if (soleOutfix) {
-        /* hs_scan -> soleOutfixBlockExec (src/runtime.c:245-280): ONE engine over the whole block,
-         * its reports are report programs (roseReportAdaptor, src/rose/match.c:611-633).  The
-         * engine runs on the DFA / NFA kernels (dfa_kernels.cu) straight from the bytecode copy;
-         * the programs are resolved on the host when the records are ordered (postprocess). */
-        if ((size_t)r->nfaInfoOffset + sizeof(NfaInfo) > h->length) {
-            delete im;
-            return HS_INVALID;
+    if (r->runtimeImpl != RUNTIME_PURE_LITERAL) {
+        /* hs_scan -> soleOutfixBlockExec (src/runtime.c:245-280), or roseBlockExec over outfixes only: every engine
+         * runs over the whole block, its reports are report programs (roseReportAdaptor / roseNfaAdaptor, src/rose/
+         * match.c:611-633).  The engines run on the DFA / NFA kernels (dfa_kernels.cu) straight from the bytecode
+         * copy, one launch per engine model; the programs are resolved on the host when the records are ordered
+         * (postprocess). */
+        struct Eng {
+            DfaParams p;
+            u32 offset;
+        };
+        std::vector<Eng> engs;
+        for (u32 q = 0; q < r->queueCount; q++) {
+            const u64 at = (u64)r->nfaInfoOffset + (u64)q * sizeof(NfaInfo);
+            if (at + sizeof(NfaInfo) > h->length) {
+                delete im;
+                return HS_INVALID;
+            }
+            NfaInfo ni;
+            memcpy(&ni, bc + at, sizeof(ni));
+            if (ni.nfaOffset % 64 || (size_t)ni.nfaOffset + sizeof(NFA) > h->length) {
+                delete im;
+                return HS_INVALID;
+            }
+            NFA nh;
+            memcpy(&nh, bc + ni.nfaOffset, sizeof(nh));
+            if ((size_t)ni.nfaOffset + nh.length > h->length) {
+                delete im;
+                return HS_INVALID;
+            }
+            Eng e;
+            const hs_error_t er = engineParams(bc + ni.nfaOffset, nh.length, &e.p);
+            if (er != HS_SUCCESS) {
+                delete im;
+                return er;
+            }
+            e.offset = ni.nfaOffset;
+            engs.push_back(e);
         }
-        NfaInfo ni;
-        memcpy(&ni, bc + r->nfaInfoOffset, sizeof(ni));
-        if (ni.nfaOffset % 64 || (size_t)ni.nfaOffset + sizeof(NFA) > h->length) {
-            delete im;
-            return HS_INVALID;
-        }
-        NFA nh;
-        memcpy(&nh, bc + ni.nfaOffset, sizeof(nh));
-        if ((size_t)ni.nfaOffset + nh.length > h->length) {
-            delete im;
-            return HS_INVALID;
-        }
-        const hs_error_t er = engineParams(bc + ni.nfaOffset, nh.length, &im->nfaParams);
-        if (er != HS_SUCCESS) {
-            delete im;
-            return er;
-        }
+        std::stable_sort(engs.begin(), engs.end(), [](const Eng &a, const Eng &b) { return a.p.kind < b.p.kind; });
         im->kind = FK_OUTFIX;
-        im->nfaOffset = ni.nfaOffset;
-        im->nfaLength = nh.length;
         im->groups = 0;
         cudaError_t e = cudaMalloc(&im->d_bc, HSB_ROUNDUP(h->length, 16));
         if (e == cudaSuccess) {
             e = cudaMemcpy(im->d_bc, bc, h->length, cudaMemcpyHostToDevice);
         }
+        std::vector<DfaEngine> table(engs.size());
+        for (size_t i = 0; i < engs.size(); i++) {
+            const DfaParams &ep = engs[i].p;
+            table[i] = {im->d_bc + engs[i].offset, ep.tableBytes, ep.states, ep.squashes, 0};
+        }
+        if (e == cudaSuccess) {
+            e = cudaMalloc(&im->d_engines, table.size() * sizeof(DfaEngine));
+        }
+        if (e == cudaSuccess) {
+            e = cudaMemcpy(im->d_engines, table.data(), table.size() * sizeof(DfaEngine), cudaMemcpyHostToDevice);
+        }
         if (e != cudaSuccess) {
             freeImage(im);
             return e == cudaErrorMemoryAllocation ? HS_NOMEM : HS_UNKNOWN_ERROR;
         }
-        im->deviceBytes = HSB_ROUNDUP(h->length, 16);
+        for (size_t i = 0; i < engs.size(); i++) {
+            const DfaParams &ep = engs[i].p;
+            if (im->engineLaunches.empty() || im->engineLaunches.back().kind != ep.kind) {
+                im->engineLaunches.push_back(ep);
+                im->engineLaunches.back().engines = im->d_engines + i;
+                im->engineLaunches.back().nengines = 0;
+            }
+            DfaParams &l = im->engineLaunches.back();
+            l.nengines++;
+            l.tableBytes = std::max(l.tableBytes, ep.tableBytes);
+            l.states = std::max(l.states, ep.states);
+            l.squashes |= ep.squashes;
+        }
+        im->deviceBytes = HSB_ROUNDUP(h->length, 16) + table.size() * sizeof(DfaEngine);
         *out = im;
         return HS_SUCCESS;
     }
@@ -1314,23 +1352,23 @@ hs_error_t launchRange(hs_scratch *s, const DevImage *im, const hs_b200_corpus *
         if (t1 < ntiles) {
             return HS_SUCCESS;
         }
-        DfaParams dp = im->nfaParams;
-        dp.corpus = c->d_data;
-        dp.readableEnd = c->readableEnd;
-        dp.blockOff = c->d_off;
-        dp.blockLen = c->d_len;
-        dp.nblocks = (u32)c->nblocks;
-        dp.uniformPitch = c->uniformPitch;
-        dp.uniformLen = c->uniformLen;
-        dp.nfa = im->d_bc + im->nfaOffset;
-        dp.out = s->d_out;
-        dp.outCap = s->outCap;
-        dp.counters = s->d_counters;
         int smCount = 0, maxSmem = 0;
         cudaDeviceGetAttribute(&smCount, cudaDevAttrMultiProcessorCount, s->device);
         cudaDeviceGetAttribute(&maxSmem, cudaDevAttrMaxSharedMemoryPerBlockOptin, s->device);
-        CUDA_TRY(launchDfa(dp, smCount, maxSmem, stream));
-        g_launches++;
+        for (DfaParams dp : im->engineLaunches) { /* every engine of one model in one launch */
+            dp.corpus = c->d_data;
+            dp.readableEnd = c->readableEnd;
+            dp.blockOff = c->d_off;
+            dp.blockLen = c->d_len;
+            dp.nblocks = (u32)c->nblocks;
+            dp.uniformPitch = c->uniformPitch;
+            dp.uniformLen = c->uniformLen;
+            dp.out = s->d_out;
+            dp.outCap = s->outCap;
+            dp.counters = s->d_counters;
+            CUDA_TRY(launchDfa(dp, smCount, maxSmem, stream));
+            g_launches++;
+        }
         return HS_SUCCESS;
     }
     ScanParams p;
@@ -2203,15 +2241,20 @@ hs_error_t hs_b200_nfa_scan_corpus(const void *nfa, size_t nfa_len, const hs_b20
     int smCount = 0, maxSmem = 0;
     cudaDeviceGetAttribute(&smCount, cudaDevAttrMultiProcessorCount, corpus->device);
     cudaDeviceGetAttribute(&maxSmem, cudaDevAttrMaxSharedMemoryPerBlockOptin, corpus->device);
-    u8 *d_nfa = nullptr;
+    u8 *d_nfa = nullptr; /* the engine's bytes, then its entry of the engine table */
     u32 *d_ctr = nullptr;
     DevMatch *d_out = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     hs_error_t rv = HS_SUCCESS;
     u32 capDev = (u32)std::min<size_t>(std::max<size_t>(cap, 1u << 16), 0xfffffff0u);
     std::vector<DevMatch> host;
-    cudaError_t e = cudaMalloc(&d_nfa, HSB_ROUNDUP(nfa_len, 16));
+    const size_t entryAt = HSB_ROUNDUP(nfa_len, 16);
+    cudaError_t e = cudaMalloc(&d_nfa, entryAt + sizeof(DfaEngine));
     if (e == cudaSuccess) e = cudaMemcpy(d_nfa, nfa, nfa_len, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) {
+        const DfaEngine entry = {d_nfa, p.tableBytes, p.states, p.squashes, 0};
+        e = cudaMemcpy(d_nfa + entryAt, &entry, sizeof(entry), cudaMemcpyHostToDevice);
+    }
     if (e == cudaSuccess) e = cudaMalloc(&d_ctr, CTR_COUNT * sizeof(u32));
     if (e == cudaSuccess) e = cudaEventCreate(&ev0);
     if (e == cudaSuccess) e = cudaEventCreate(&ev1);
@@ -2226,7 +2269,8 @@ hs_error_t hs_b200_nfa_scan_corpus(const void *nfa, size_t nfa_len, const hs_b20
         p.nblocks = (u32)corpus->nblocks;
         p.uniformPitch = corpus->uniformPitch;
         p.uniformLen = corpus->uniformLen;
-        p.nfa = d_nfa;
+        p.engines = reinterpret_cast<const DfaEngine *>(d_nfa + entryAt);
+        p.nengines = 1;
         p.out = d_out;
         p.outCap = capDev;
         p.counters = d_ctr;

@@ -57,10 +57,10 @@ __device__ __forceinline__ u32 emitDfaMatch(const DfaParams &p, u32 cursor, u32 
 }
 
 /* struct report_list {u32 count; ReportID report[]} at NFA offset `off` */
-__device__ u32 emitReportList(const DfaParams &p, u32 cursor, u32 off, u32 block, u64 to) {
-    const u32 n = g32(p.nfa + off);
+__device__ u32 emitReportList(const DfaParams &p, const u8 *nfa, u32 cursor, u32 off, u32 block, u64 to) {
+    const u32 n = g32(nfa + off);
     for (u32 i = 0; i < n; i++) {
-        cursor = emitDfaMatch(p, cursor, g32(p.nfa + off + 4 + 4 * i), block, to);
+        cursor = emitDfaMatch(p, cursor, g32(nfa + off + 4 + 4 * i), block, to);
     }
     return cursor;
 }
@@ -223,8 +223,9 @@ template <int W> struct StOps<WideSt<W>> {
 };
 
 /* LimEx report list: ReportID[] terminated by MO_INVALID_IDX (limexRunReports, limex_runtime.h:90-103) */
-__device__ HSB_NOINLINE u32 emitLimexReports(const DfaParams &p, u32 cursor, u32 listOff, u32 block, u64 to) {
-    const u8 *lx = p.nfa + sizeof(NFA);
+__device__ HSB_NOINLINE u32 emitLimexReports(const DfaParams &p, const u8 *nfa, u32 cursor, u32 listOff, u32 block,
+                                             u64 to) {
+    const u8 *lx = nfa + sizeof(NFA);
     for (u32 i = 0;; i++) {
         const u32 id = g32(lx + listOff + 4 * i);
         if (id == MO_INVALID_IDX) {
@@ -238,9 +239,9 @@ __device__ HSB_NOINLINE u32 emitLimexReports(const DfaParams &p, u32 cursor, u32
 /* accepts of the states in `found` through an NFAAccept table (PROCESS_ACCEPTS_IMPL_FN,
  * limex_common_impl.h:116-163; the squash of PROCESS_ACCEPTS_FN is dead code there) */
 template <class ST>
-__device__ HSB_NOINLINE u32 emitLimexAccepts(const DfaParams &p, u32 cursor, ST found, ST mask, u32 tableOff,
-                                             u32 block, u64 to) {
-    const u8 *lx = p.nfa + sizeof(NFA);
+__device__ HSB_NOINLINE u32 emitLimexAccepts(const DfaParams &p, const u8 *nfa, u32 cursor, ST found, ST mask,
+                                             u32 tableOff, u32 block, u64 to) {
+    const u8 *lx = nfa + sizeof(NFA);
     StOps<ST>::forEach(found, [&](const u32 bit) {
         const u32 idx = StOps<ST>::rank(mask, bit);
         const u8 *a = lx + tableOff + idx * (u32)sizeof(NFAAccept);
@@ -248,7 +249,7 @@ __device__ HSB_NOINLINE u32 emitLimexAccepts(const DfaParams &p, u32 cursor, ST 
         if (__ldg(a + offsetof(NFAAccept, single_report))) {
             cursor = emitDfaMatch(p, cursor, reports, block, to);
         } else {
-            cursor = emitLimexReports(p, cursor, reports, block, to);
+            cursor = emitLimexReports(p, nfa, cursor, reports, block, to);
         }
     });
     return cursor;
@@ -389,11 +390,12 @@ struct DfaConsts {
 /* reports of a state that was just entered at offset `to` (doComplexReport, mcclellan.c:43-91;
  * fireReports, sheng_impl.h:116-155).  what = the one report of a single-report engine, else
  * the offset of the state's aux record.  Returns the lane's record cursor. */
-__device__ HSB_NOINLINE u32 emitAccept(const DfaParams &p, u32 cursor, u32 single, u32 what, u32 block, u64 to) {
+__device__ HSB_NOINLINE u32 emitAccept(const DfaParams &p, const u8 *nfa, u32 cursor, u32 single, u32 what, u32 block,
+                                       u64 to) {
     if (single) {
         return emitDfaMatch(p, cursor, what, block, to);
     }
-    return emitReportList(p, cursor, g32(p.nfa + what), block, to);
+    return emitReportList(p, nfa, cursor, g32(nfa + what), block, to);
 }
 
 template <int ENGINE, int SMEM_TABLE, int CH, int ILP>
@@ -401,166 +403,174 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
     HSB_DYNAMIC_SMEM(smem);
     typedef DfaTile<CH> Tile;
     const u32 lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-    const u8 *eng = p.nfa + sizeof(NFA); /* struct mcclellan / struct sheng */
-    const u8 *succG = eng + sizeof(McClellan);
-    DfaConsts k;
-    k.as = 0;
-    k.shermanOffset = 0;
-    k.shermanLimit = 0xffffffffu;
-    k.acceptLimit8 = 0;
     typedef typename WalkState<ENGINE>::type ST;
     typedef typename LimexLayout<ST>::Nfa LxNfa;
     typedef typename LimexLayout<ST>::Exc LxExc;
     typedef StOps<ST> Ops;
     constexpr bool LIMEX = ENGINE >= ENG_LIMEX32;
     constexpr bool WIDE = ENGINE >= ENG_LIMEX128; /* state sets of several 64-bit words */
+    /* the engine the CTA runs (DfaParams.engines[current]) and its constants.  The LimEx walks read its bytes back
+     * from the table where a report needs them rather than hold them in registers through the walk (measured
+     * faster there; the DFA walks, whose accepts are frequent, are faster with them in a register). */
+    u32 current = 0xffffffffu;
+    const u8 *dfaBytes = nullptr;
+    auto engineBytes = [&]() -> const u8 * { return LIMEX ? p.engines[current].nfa : dfaBytes; }; /* struct NFA */
+    u32 squashes = 0;
+    DfaConsts k;
     ST lxAccept = Ops::zero(), lxAcceptEod = Ops::zero(), lxStart = Ops::zero();
-    if (LIMEX) {
-        /* eng = struct LimExNFA32 ... 512; a top at offset 0 switches `init` on (moNfaTop) */
-        lxStart = Ops::load(eng + offsetof(LxNfa, init));
-        k.start = 0;
-        k.single = 0;
-        k.report = 0;
-        k.auxOffset = 0;
-        k.auxSize = 0;
-        k.stateMask = 0xffffffffu;
-        lxAccept = Ops::load(eng + offsetof(LxNfa, accept));
-        lxAcceptEod = Ops::load(eng + offsetof(LxNfa, acceptAtEOD));
-    } else if (ENGINE == ENG_SHENG) {
-        k.start = __ldg(eng + offsetof(Sheng, anchored));
-        k.single = __ldg(eng + offsetof(Sheng, flags)) & SHENG_FLAG_SINGLE_REPORT;
-        k.report = g32(eng + offsetof(Sheng, report));
-        k.auxOffset = g32(eng + offsetof(Sheng, aux_offset));
-        k.auxSize = (u32)sizeof(SstateAux);
-        k.stateMask = SHENG_STATE_MASK;
-    } else {
-        k.as = __ldg(eng + offsetof(McClellan, alphaShift));
-        k.single = __ldg(eng + offsetof(McClellan, flags)) & MCCLELLAN_FLAG_SINGLE;
-        k.report = g32(eng + offsetof(McClellan, arb_report));
-        k.start = g16(eng + offsetof(McClellan, start_anchored));
-        k.auxOffset = g32(eng + offsetof(McClellan, aux_offset));
-        k.shermanOffset = g32(eng + offsetof(McClellan, sherman_offset));
-        if (ENGINE == ENG_MCC16) {
-            k.shermanLimit = g16(eng + offsetof(McClellan, sherman_limit));
-        }
-        k.acceptLimit8 = g16(eng + offsetof(McClellan, accept_limit_8));
-        k.auxSize = (u32)sizeof(MStateAux);
-        k.stateMask = 0xffffffffu;
-    }
-    u32 tabArea;
-    if (LIMEX) {
-        /* (32- and 64-state models) reach mask by byte value (reach[reachMap[b]]), then ONE row of four ST per state i:
-         *   [0] its limited successors: OR over the shifts k with bit i of shift[k] of 1 << (i + shiftAmount[k])
-         *   [1] its exception's successors, [2] its squash mask (all ones unless the exception squashes:
-         *   LIMEX_SQUASH_CYCLIC / _REPORT), [3] its exception's report list
-         * so a byte costs work in proportion to the states that are ON, not eight shift-and-mask rounds */
-        const u8 *reach = eng + sizeof(LxNfa);
-        const ST excMask = Ops::load(eng + offsetof(LxNfa, exceptionMask));
-        const u32 nshift = g32(eng + offsetof(LxNfa, shiftCount));
-        const u8 *exc = eng + g32(eng + offsetof(LxNfa, exceptionOffset));
-        /* row of state i: limited successors, exception successors, squash mask, report list */
-        auto rowOf = [&](const u32 i, ST &lim, ST &local, ST &keep, u32 &rep) {
-            lim = Ops::zero(), local = Ops::zero(), keep = Ops::ones(), rep = MO_INVALID_IDX;
-            for (u32 q = 0; q < nshift && q < 8; q++) {
-                if (Ops::test(Ops::load(eng + offsetof(LxNfa, shift) + sizeof(ST) * q), i)) {
-                    lim = Ops::bor(lim, Ops::shiftedBit(i, __ldg(eng + offsetof(LxNfa, shiftAmount) + q)));
-                }
-            }
-            if (Ops::test(excMask, i)) {
-                const u8 *x = exc + Ops::rank(excMask, i) * (u32)sizeof(LxExc);
-                const u32 kind = __ldg(x + offsetof(LxExc, hasSquash));
-                local = Ops::load(x + offsetof(LxExc, successors));
-                rep = g32(x + offsetof(LxExc, reports));
-                if (kind == LIMEX_SQUASH_CYCLIC || kind == LIMEX_SQUASH_REPORT) {
-                    keep = Ops::load(x + offsetof(LxExc, squash));
-                }
-            }
-        };
-        if constexpr (WIDE) {
-            typedef LimexTable<ST> T;
-            for (u32 i = threadIdx.x; i < 256; i += blockDim.x) {
-                Ops::storeChunks(reinterpret_cast<uint4 *>(smem + T::REACH), 256, i,
-                                 Ops::load(reach + sizeof(ST) * __ldg(eng + offsetof(LxNfa, reachMap) + i)));
-            }
-            for (u32 i = threadIdx.x; i < T::STATES; i += blockDim.x) {
-                ST lim, local, keep;
-                u32 rep;
-                rowOf(i, lim, local, keep, rep);
-                Ops::storeChunks(reinterpret_cast<uint4 *>(smem + T::LOCAL), T::STATES, i, local);
-                Ops::storeChunks(reinterpret_cast<uint4 *>(smem + T::KEEP), T::STATES, i, keep);
-                reinterpret_cast<u32 *>(smem + T::REP)[i] = rep;
-            }
-            for (u32 i = threadIdx.x; i < 9; i += blockDim.x) { /* shift masks 0..7, then the exception mask */
-                reinterpret_cast<ST *>(smem + T::SHIFT)[i] =
-                    i < 8 ? (i < nshift ? Ops::load(eng + offsetof(LxNfa, shift) + sizeof(ST) * i) : Ops::zero()) : excMask;
-            }
-        } else {
-            ST *d = reinterpret_cast<ST *>(smem);
-            for (u32 i = threadIdx.x; i < 256; i += blockDim.x) {
-                d[i] = Ops::load(reach + sizeof(ST) * __ldg(eng + offsetof(LxNfa, reachMap) + i));
-            }
-            ST *rows = d + 256;
-            for (u32 i = threadIdx.x; i < 8 * sizeof(ST); i += blockDim.x) {
-                ST lim, local, keep;
-                u32 rep;
-                rowOf(i, lim, local, keep, rep);
-                rows[4 * i + 0] = lim;
-                rows[4 * i + 1] = local;
-                rows[4 * i + 2] = keep;
-                rows[4 * i + 3] = Ops::fromU32(rep);
-            }
-        }
-        tabArea = LimexTable<ST>::BYTES;
-    } else if (ENGINE == ENG_SHENG) {
-        /* [byte c][copy r][16 successor bytes, the one of state s at position (s + 4c) & 15] */
-        for (u32 i = threadIdx.x; i < SHENG_TABLE_BYTES; i += blockDim.x) {
-            const u32 c = i >> 7;
-            smem[i] = __ldg(eng + c * 16 + (((i & 15) - 4 * c) & 15));
-        }
-        tabArea = SHENG_TABLE_BYTES;
-    } else if (ENGINE == ENG_MCC8) {
-        const u32 states = g16(eng + offsetof(McClellan, state_count));
-        for (u32 i = threadIdx.x; i < states * 256; i += blockDim.x) {
-            const u32 cp = __ldg(eng + offsetof(McClellan, remap) + (i & 255));
-            smem[i] = __ldg(succG + ((i >> 8) << k.as) + cp);
-        }
-        tabArea = states * 256;
-    } else {
-        for (u32 i = threadIdx.x; i < 256; i += blockDim.x) {
-            smem[i] = __ldg(eng + offsetof(McClellan, remap) + i);
-        }
-        tabArea = 256;
-        if (SMEM_TABLE) {
-            u32 *d = reinterpret_cast<u32 *>(smem + 256);
-            const u32 *g = reinterpret_cast<const u32 *>(succG);
-            for (u32 i = threadIdx.x; i < (p.tableBytes + 3) / 4; i += blockDim.x) {
-                d[i] = __ldg(g + i);
-            }
-            tabArea += HSB_ROUNDUP(p.tableBytes, 16);
-        }
-    }
-    __syncthreads();
-    u8 *const tile = smem + tabArea + warp * (ILP * Tile::WARP_BYTES);
+    u8 *const tile = smem + p.tableArea + warp * (ILP * Tile::WARP_BYTES);
     const u8 *const myRow = tile + lane * Tile::ROW;
-    const u16 *succ16 = reinterpret_cast<const u16 *>(SMEM_TABLE ? smem + 256 : succG);
+    const u16 *succ16 = nullptr;
     const u32 copyOff = (lane & 7) * 16; /* Sheng: this lane's copy of a row */
-
     const ST *lxReach = reinterpret_cast<const ST *>(smem);
     const ST *lxRows = lxReach + 256;
     ST lxLim0 = Ops::zero(), lxLocal0 = Ops::zero(), lxKeep0 = Ops::ones();
     bool lxRow0Plain = false; /* state 0 raises no reports: its row can be applied without the loop */
-    if (LIMEX && !WIDE) { /* (the wide models read it from shared memory like every other row) */
-        lxLim0 = lxRows[0];
-        lxLocal0 = lxRows[1];
-        lxKeep0 = lxRows[2];
-        lxRow0Plain = Ops::low32(lxRows[3]) == MO_INVALID_IDX;
-    }
     u32 lxShiftCount = 0;
     u64 lxShiftAmounts = 0; /* shiftAmount[0..7], one byte each */
-    if (WIDE) {
-        lxShiftCount = min(g32(eng + offsetof(LxNfa, shiftCount)), 8u);
-        lxShiftAmounts = (u64)g32(eng + offsetof(LxNfa, shiftAmount)) | ((u64)g32(eng + offsetof(LxNfa, shiftAmount) + 4) << 32);
-    }
+    /* Switch the whole CTA to engine e: its constants, and its tables in shared memory (the caller has made sure
+     * that no warp still reads the previous engine's) */
+    auto loadEngine = [&](const u32 e) {
+        const DfaEngine en = p.engines[e];
+        dfaBytes = en.nfa;
+        const u8 *const eng = en.nfa + sizeof(NFA); /* struct mcclellan / struct sheng / LimExNFA* */
+        const u8 *const succG = eng + sizeof(McClellan);
+        squashes = en.squashes;
+        k.as = 0;
+        k.shermanOffset = 0;
+        k.shermanLimit = 0xffffffffu;
+        k.acceptLimit8 = 0;
+        if (LIMEX) {
+            /* eng = struct LimExNFA32 ... 512; a top at offset 0 switches `init` on (moNfaTop) */
+            lxStart = Ops::load(eng + offsetof(LxNfa, init));
+            k.start = 0;
+            k.single = 0;
+            k.report = 0;
+            k.auxOffset = 0;
+            k.auxSize = 0;
+            k.stateMask = 0xffffffffu;
+            lxAccept = Ops::load(eng + offsetof(LxNfa, accept));
+            lxAcceptEod = Ops::load(eng + offsetof(LxNfa, acceptAtEOD));
+        } else if (ENGINE == ENG_SHENG) {
+            k.start = __ldg(eng + offsetof(Sheng, anchored));
+            k.single = __ldg(eng + offsetof(Sheng, flags)) & SHENG_FLAG_SINGLE_REPORT;
+            k.report = g32(eng + offsetof(Sheng, report));
+            k.auxOffset = g32(eng + offsetof(Sheng, aux_offset));
+            k.auxSize = (u32)sizeof(SstateAux);
+            k.stateMask = SHENG_STATE_MASK;
+        } else {
+            k.as = __ldg(eng + offsetof(McClellan, alphaShift));
+            k.single = __ldg(eng + offsetof(McClellan, flags)) & MCCLELLAN_FLAG_SINGLE;
+            k.report = g32(eng + offsetof(McClellan, arb_report));
+            k.start = g16(eng + offsetof(McClellan, start_anchored));
+            k.auxOffset = g32(eng + offsetof(McClellan, aux_offset));
+            k.shermanOffset = g32(eng + offsetof(McClellan, sherman_offset));
+            if (ENGINE == ENG_MCC16) {
+                k.shermanLimit = g16(eng + offsetof(McClellan, sherman_limit));
+            }
+            k.acceptLimit8 = g16(eng + offsetof(McClellan, accept_limit_8));
+            k.auxSize = (u32)sizeof(MStateAux);
+            k.stateMask = 0xffffffffu;
+        }
+        if (LIMEX) {
+            /* (32- and 64-state models) reach mask by byte value (reach[reachMap[b]]), then ONE row of four ST per state i:
+             *   [0] its limited successors: OR over the shifts k with bit i of shift[k] of 1 << (i + shiftAmount[k])
+             *   [1] its exception's successors, [2] its squash mask (all ones unless the exception squashes:
+             *   LIMEX_SQUASH_CYCLIC / _REPORT), [3] its exception's report list
+             * so a byte costs work in proportion to the states that are ON, not eight shift-and-mask rounds */
+            const u8 *reach = eng + sizeof(LxNfa);
+            const ST excMask = Ops::load(eng + offsetof(LxNfa, exceptionMask));
+            const u32 nshift = g32(eng + offsetof(LxNfa, shiftCount));
+            const u8 *exc = eng + g32(eng + offsetof(LxNfa, exceptionOffset));
+            /* row of state i: limited successors, exception successors, squash mask, report list */
+            auto rowOf = [&](const u32 i, ST &lim, ST &local, ST &keep, u32 &rep) {
+                lim = Ops::zero(), local = Ops::zero(), keep = Ops::ones(), rep = MO_INVALID_IDX;
+                for (u32 q = 0; q < nshift && q < 8; q++) {
+                    if (Ops::test(Ops::load(eng + offsetof(LxNfa, shift) + sizeof(ST) * q), i)) {
+                        lim = Ops::bor(lim, Ops::shiftedBit(i, __ldg(eng + offsetof(LxNfa, shiftAmount) + q)));
+                    }
+                }
+                if (Ops::test(excMask, i)) {
+                    const u8 *x = exc + Ops::rank(excMask, i) * (u32)sizeof(LxExc);
+                    const u32 kind = __ldg(x + offsetof(LxExc, hasSquash));
+                    local = Ops::load(x + offsetof(LxExc, successors));
+                    rep = g32(x + offsetof(LxExc, reports));
+                    if (kind == LIMEX_SQUASH_CYCLIC || kind == LIMEX_SQUASH_REPORT) {
+                        keep = Ops::load(x + offsetof(LxExc, squash));
+                    }
+                }
+            };
+            if constexpr (WIDE) {
+                typedef LimexTable<ST> T;
+                for (u32 i = threadIdx.x; i < 256; i += blockDim.x) {
+                    Ops::storeChunks(reinterpret_cast<uint4 *>(smem + T::REACH), 256, i,
+                                     Ops::load(reach + sizeof(ST) * __ldg(eng + offsetof(LxNfa, reachMap) + i)));
+                }
+                for (u32 i = threadIdx.x; i < T::STATES; i += blockDim.x) {
+                    ST lim, local, keep;
+                    u32 rep;
+                    rowOf(i, lim, local, keep, rep);
+                    Ops::storeChunks(reinterpret_cast<uint4 *>(smem + T::LOCAL), T::STATES, i, local);
+                    Ops::storeChunks(reinterpret_cast<uint4 *>(smem + T::KEEP), T::STATES, i, keep);
+                    reinterpret_cast<u32 *>(smem + T::REP)[i] = rep;
+                }
+                for (u32 i = threadIdx.x; i < 9; i += blockDim.x) { /* shift masks 0..7, then the exception mask */
+                    reinterpret_cast<ST *>(smem + T::SHIFT)[i] =
+                        i < 8 ? (i < nshift ? Ops::load(eng + offsetof(LxNfa, shift) + sizeof(ST) * i) : Ops::zero()) : excMask;
+                }
+            } else {
+                ST *d = reinterpret_cast<ST *>(smem);
+                for (u32 i = threadIdx.x; i < 256; i += blockDim.x) {
+                    d[i] = Ops::load(reach + sizeof(ST) * __ldg(eng + offsetof(LxNfa, reachMap) + i));
+                }
+                ST *rows = d + 256;
+                for (u32 i = threadIdx.x; i < 8 * sizeof(ST); i += blockDim.x) {
+                    ST lim, local, keep;
+                    u32 rep;
+                    rowOf(i, lim, local, keep, rep);
+                    rows[4 * i + 0] = lim;
+                    rows[4 * i + 1] = local;
+                    rows[4 * i + 2] = keep;
+                    rows[4 * i + 3] = Ops::fromU32(rep);
+                }
+            }
+        } else if (ENGINE == ENG_SHENG) {
+            /* [byte c][copy r][16 successor bytes, the one of state s at position (s + 4c) & 15] */
+            for (u32 i = threadIdx.x; i < SHENG_TABLE_BYTES; i += blockDim.x) {
+                const u32 c = i >> 7;
+                smem[i] = __ldg(eng + c * 16 + (((i & 15) - 4 * c) & 15));
+            }
+        } else if (ENGINE == ENG_MCC8) {
+            const u32 states = g16(eng + offsetof(McClellan, state_count));
+            for (u32 i = threadIdx.x; i < states * 256; i += blockDim.x) {
+                const u32 cp = __ldg(eng + offsetof(McClellan, remap) + (i & 255));
+                smem[i] = __ldg(succG + ((i >> 8) << k.as) + cp);
+            }
+        } else {
+            for (u32 i = threadIdx.x; i < 256; i += blockDim.x) {
+                smem[i] = __ldg(eng + offsetof(McClellan, remap) + i);
+            }
+            if (SMEM_TABLE) {
+                u32 *d = reinterpret_cast<u32 *>(smem + 256);
+                const u32 *g = reinterpret_cast<const u32 *>(succG);
+                for (u32 i = threadIdx.x; i < (en.tableBytes + 3) / 4; i += blockDim.x) {
+                    d[i] = __ldg(g + i);
+                }
+            }
+        }
+        __syncthreads();
+        succ16 = reinterpret_cast<const u16 *>(SMEM_TABLE ? smem + 256 : succG);
+        if (LIMEX && !WIDE) { /* (the wide models read it from shared memory like every other row) */
+            lxLim0 = lxRows[0];
+            lxLocal0 = lxRows[1];
+            lxKeep0 = lxRows[2];
+            lxRow0Plain = Ops::low32(lxRows[3]) == MO_INVALID_IDX;
+        }
+        if (WIDE) {
+            lxShiftCount = min(g32(eng + offsetof(LxNfa, shiftCount)), 8u);
+            lxShiftAmounts = (u64)g32(eng + offsetof(LxNfa, shiftAmount)) | ((u64)g32(eng + offsetof(LxNfa, shiftAmount) + 4) << 32);
+        }
+    };
     u32 cursor = 0; /* this lane's next record slot (emitDfaMatch) */
     /* one input byte: byte j of data word w, at block offset pos.  DFAs: returns true when the
      * state entered accepts.  LimEx (LOOP_NOACCEL_FN, limex_runtime_impl.h:209-243): the states
@@ -585,10 +595,10 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
             Ops::forEach(Ops::band(s, tShift[8]), [&](const u32 bit) {
                 const u32 rep = reinterpret_cast<const u32 *>(smem + T::REP)[bit];
                 if (rep != MO_INVALID_IDX && pos != 0) {
-                    cursor = emitLimexReports(p, cursor, rep, blk, pos);
+                    cursor = emitLimexReports(p, engineBytes(), cursor, rep, blk, pos);
                 }
                 local = Ops::bor(local, Ops::loadChunks(reinterpret_cast<const uint4 *>(smem + T::LOCAL), T::STATES, bit));
-                if (p.squashes) {
+                if (squashes) {
                     keep = Ops::band(keep, Ops::loadChunks(reinterpret_cast<const uint4 *>(smem + T::KEEP), T::STATES, bit));
                 }
             });
@@ -612,7 +622,7 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
                 const ST *e = lxRows + 4 * bit;
                 const u32 rep = Ops::low32(e[3]);
                 if (rep != MO_INVALID_IDX && pos != 0) {
-                    cursor = emitLimexReports(p, cursor, rep, blk, pos);
+                    cursor = emitLimexReports(p, engineBytes(), cursor, rep, blk, pos);
                 }
                 lim = Ops::bor(lim, e[0]);
                 local = Ops::bor(local, e[1]);
@@ -633,7 +643,9 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
             if (s < k.shermanLimit) {
                 e = SMEM_TABLE ? succ16[(s << k.as) + cp] : __ldg(succ16 + (s << k.as) + cp);
             } else {
-                e = shermanNext(p.nfa, k.shermanOffset, k.shermanLimit, s, cp, reinterpret_cast<const u16 *>(succG),
+                const u8 *nfa = engineBytes();
+                e = shermanNext(nfa, k.shermanOffset, k.shermanLimit, s, cp,
+                                reinterpret_cast<const u16 *>(nfa + sizeof(NFA) + sizeof(McClellan)),
                                 k.as);
             }
             s = e & MCC_STATE_MASK;
@@ -648,10 +660,26 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
     };
 
     /* a warp takes 32 * ILP consecutive blocks at a time; lane t owns blocks t, t + 32, ...
-     * of the group: ILP independent state chains in one instruction stream */
+     * of the group: ILP independent state chains in one instruction stream.  The work of a launch is
+     * every engine over every group, in rounds of one engine and nwarps consecutive groups (a warp each),
+     * engine-major; CTA c takes rounds c, c + gridDim.x, ... -- with one engine the round-robin over the
+     * groups it always was -- and so meets the engines in order, building each one's tables once. */
     const u32 perGroup = 32 * ILP;
     const u32 ngroups = (p.nblocks + perGroup - 1) / perGroup;
-    for (u32 g = blockIdx.x * nwarps + warp; g < ngroups; g += gridDim.x * nwarps) {
+    const u32 rounds = (ngroups + nwarps - 1) / nwarps; /* of one engine */
+    for (u32 round = blockIdx.x; round < rounds * p.nengines; round += gridDim.x) {
+        const u32 e = round / rounds;
+        if (e != current) { /* (uniform across the CTA: every warp walks the same rounds) */
+            if (current != 0xffffffffu) {
+                __syncthreads();
+            }
+            current = e;
+            loadEngine(e);
+        }
+        const u32 g = (round - e * rounds) * nwarps + warp;
+        if (g >= ngroups) {
+            continue;
+        }
         u32 b[ILP], len[ILP];
         ST s[ILP];
         u64 off[ILP];
@@ -734,7 +762,7 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
 #pragma unroll
                         for (int u = 0; u < ILP; u++) {
                             if (step(w[u][j >> 2], j & 3, s[u], done + c * 16 + j, b[u])) {
-                                cursor = emitAccept(p, cursor, k.single, acceptWhat(s[u]), b[u], (u64)done + c * 16 + j + 1);
+                                cursor = emitAccept(p, engineBytes(), cursor, k.single, acceptWhat(s[u]), b[u], (u64)done + c * 16 + j + 1);
                             }
                         }
                     }
@@ -768,7 +796,7 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
 #pragma unroll
                         for (u32 j = 0; j < 16; j++) {
                             if (step(w[j >> 2], j & 3, s[u], done + cc * 16 + j, b[u])) {
-                                cursor = emitAccept(p, cursor, k.single, acceptWhat(s[u]), b[u], (u64)done + cc * 16 + j + 1);
+                                cursor = emitAccept(p, engineBytes(), cursor, k.single, acceptWhat(s[u]), b[u], (u64)done + cc * 16 + j + 1);
                             }
                         }
                         live[u] = !dead(s[u]);
@@ -780,7 +808,7 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
 #pragma unroll 1
                         for (u32 j = 0; j < m; j++) {
                             if (step(w[j >> 2] >> (8 * (j & 3)), 0, s[u], done + cc * 16 + j, b[u])) {
-                                cursor = emitAccept(p, cursor, k.single, acceptWhat(s[u]), b[u], (u64)done + cc * 16 + j + 1);
+                                cursor = emitAccept(p, engineBytes(), cursor, k.single, acceptWhat(s[u]), b[u], (u64)done + cc * 16 + j + 1);
                             }
                         }
                         live[u] = !dead(s[u]);
@@ -797,20 +825,24 @@ __global__ void __launch_bounds__(StagedThreads<ENGINE>::N, 1) dfaStagedKernel(c
                     /* STREAM_FN's closing accept check (only if the block had bytes to stream),
                      * then nfaExecLimEx*_testEOD (limex_common_impl.h:192-218) */
                     if (len[u] && Ops::any(Ops::band(s[u], lxAccept))) {
-                        cursor = emitLimexAccepts<ST>(p, cursor, Ops::band(s[u], lxAccept), lxAccept,
-                                                      g32(eng + offsetof(LxNfa, acceptOffset)), b[u], len[u]);
+                        const u8 *nfa = engineBytes();
+                        cursor = emitLimexAccepts<ST>(p, nfa, cursor, Ops::band(s[u], lxAccept), lxAccept,
+                                                      g32(nfa + sizeof(NFA) + offsetof(LxNfa, acceptOffset)), b[u], len[u]);
                     }
                     if (Ops::any(Ops::band(s[u], lxAcceptEod))) {
-                        cursor = emitLimexAccepts<ST>(p, cursor, Ops::band(s[u], lxAcceptEod), lxAcceptEod,
-                                                      g32(eng + offsetof(LxNfa, acceptEodOffset)), b[u], len[u]);
+                        const u8 *nfa = engineBytes();
+                        cursor = emitLimexAccepts<ST>(p, nfa, cursor, Ops::band(s[u], lxAcceptEod), lxAcceptEod,
+                                                      g32(nfa + sizeof(NFA) + offsetof(LxNfa, acceptEodOffset)), b[u],
+                                                      len[u]);
                     }
                 }
             } else if (b[u] < p.nblocks) {
                 const u32 eodOff = ENGINE == ENG_SHENG ? (u32)offsetof(SstateAux, accept_eod)
                                                        : (u32)offsetof(MStateAux, accept_eod);
-                const u32 eod = g32(p.nfa + k.auxOffset + k.auxSize * (Ops::low32(s[u]) & k.stateMask) + eodOff);
+                const u8 *nfa = engineBytes();
+                const u32 eod = g32(nfa + k.auxOffset + k.auxSize * (Ops::low32(s[u]) & k.stateMask) + eodOff);
                 if (eod) {
-                    cursor = emitReportList(p, cursor, eod, b[u], len[u]);
+                    cursor = emitReportList(p, nfa, cursor, eod, b[u], len[u]);
                 }
             }
         }
@@ -827,7 +859,8 @@ cudaError_t launchStaged(const DfaParams &p, int smCount, size_t tableBytes, cud
     const bool two = p.ilp == 2 && ENGINE < ENG_LIMEX128; /* (the wide models walk one block per lane) */
     const size_t tiles = (size_t)(threads / 32) * (two ? 2 * DfaTile<64>::WARP_BYTES : DfaTile<128>::WARP_BYTES);
     const u64 groups = ((u64)p.nblocks + (two ? 63 : 31)) / (two ? 64 : 32);
-    const int grid = (int)std::min<u64>((u64)smCount, (groups + threads / 32 - 1) / (threads / 32));
+    const u64 rounds = (groups + threads / 32 - 1) / (threads / 32) * p.nengines; /* (the kernel's) */
+    const int grid = (int)std::min<u64>((u64)smCount, rounds);
     void (*kern)(const DfaParams) =
         two ? dfaStagedKernel<ENGINE, SMEM_TABLE, 64, 2> : dfaStagedKernel<ENGINE, SMEM_TABLE, 128, 1>;
     const size_t smem = tableBytes + tiles;
@@ -835,14 +868,16 @@ cudaError_t launchStaged(const DfaParams &p, int smCount, size_t tableBytes, cud
     if (e != cudaSuccess) {
         return e;
     }
-    HSB_LAUNCH(kern, grid, threads, smem, stream, p);
+    DfaParams q = p;
+    q.tableArea = (u32)tableBytes; /* the tiles follow the largest engine's tables */
+    HSB_LAUNCH(kern, grid, threads, smem, stream, q);
     return cudaGetLastError();
 }
 
 } // namespace
 
 cudaError_t launchDfa(const DfaParams &p, int smCount, int maxSmem, cudaStream_t stream) {
-    if (!p.nblocks) {
+    if (!p.nblocks || !p.nengines) {
         return cudaSuccess;
     }
     const size_t tilesMax = 32 * 2 * DfaTile<64>::WARP_BYTES;

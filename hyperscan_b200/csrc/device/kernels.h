@@ -179,8 +179,18 @@ cudaError_t launchStreamAssemble(u8 *corpus, const u8 *hist, u32 nstreams, u32 p
 cudaError_t launchStreamAdvance(const u8 *corpus, u8 *hist, u64 *offsets, const u32 *lens, u32 uniformLen,
                                 u32 nstreams, u32 pitch, u32 histReq, cudaStream_t stream);
 
-/* DFA engines in block mode (dfa_kernels.cu): McClellan 8 / 16, Sheng -- the engine's
- * own bytes (struct NFA first) in device memory, one thread per block. */
+/* One engine of a DFA / NFA launch: its own bytes (struct NFA first) in device memory. */
+struct DfaEngine {
+    const u8 *nfa;
+    u32 tableBytes;  /* McClellan: bytes of the successor table (staged in shared memory if it fits) */
+    u32 states;      /* McClellan-8: state_count (<= 256): rows of the byte-indexed table built in shared memory */
+    u32 squashes;    /* LimEx: some exception squashes (LIMEX_SQUASH_CYCLIC / _REPORT): the kernel reads the squash masks */
+    u32 pad;
+};
+
+/* DFA / NFA engines in block mode (dfa_kernels.cu): McClellan 8 / 16, Sheng, LimEx-32 ... -512, one thread per
+ * block.  One launch runs every engine of the table over every block; they are all of one model (`kind`), and
+ * tableBytes / states / squashes are the largest (any) over them, which size the launch's shared memory. */
 struct DfaParams {
     const u8 *corpus;
     u64 readableEnd;
@@ -188,12 +198,14 @@ struct DfaParams {
     const u32 *blockLen;
     u32 nblocks;
     u32 uniformPitch, uniformLen;
-    const u8 *nfa;
-    u32 kind;        /* NFA.type: NFA_MCCLELLAN_8 / NFA_MCCLELLAN_16 / NFA_SHENG */
-    u32 tableBytes;  /* McClellan: bytes of the successor table (staged in shared memory if it fits) */
+    const DfaEngine *engines; /* device memory */
+    u32 nengines;
+    u32 kind;        /* NFA.type: NFA_MCCLELLAN_8 / NFA_MCCLELLAN_16 / NFA_SHENG / NFA_LIMEX_* */
+    u32 tableBytes;
     u32 ilp;         /* blocks walked by one lane at a time: 1 or 2 (runtime option dfa_ilp) */
-    u32 states;      /* McClellan-8: state_count (<= 256): rows of the byte-indexed table built in shared memory */
-    u32 squashes;    /* LimEx: some exception squashes (LIMEX_SQUASH_CYCLIC / _REPORT): the kernel reads the squash masks */
+    u32 states;
+    u32 squashes;
+    u32 tableArea;   /* set by launchDfa: shared-memory bytes of the tables, the tiles follow */
     DevMatch *out;   /* {report, block, offset after the last byte} */
     u32 outCap;
     u32 *counters;   /* CTR_MATCHES */

@@ -5,6 +5,7 @@
 #include <cstring>
 
 #include "api_internal.h"
+#include "rose_build.h"
 
 namespace hsb {
 
@@ -16,6 +17,60 @@ namespace hsb {
  * runProgram) does not implement -- the state-carrying ones of
  * roseRunProgram_l: PUSH_DELAYED, CATCH_UP*, SOM_*, TRIGGER_SUFFIX, REPORT_CHAIN,
  * REPORT_SOM*, SET_LOGICAL, SET_COMBINATION, FLUSH_COMBINATION, SET_EXHAUST. */
+bool outfixesOnly(const RoseEngine *r, u32 bcLen) {
+    const u32 n = r->queueCount;
+    const BoundaryReports &br = r->boundary;
+    if (r->runtimeImpl != RUNTIME_FULL_ROSE || r->mode != MODE_BLOCK || !n || r->activeArrayCount != n ||
+        r->outfixBeginQueue != 0 || r->outfixEndQueue != n || r->leftfixBeginQueue != n || !r->nfaInfoOffset ||
+        r->initMpvNfa != 0xffffffffu || r->hasSom || r->somLocationCount || r->somRevCount || r->amatcherOffset ||
+        r->ematcherOffset || r->fmatcherOffset || r->drmatcherOffset || r->sbmatcherOffset || r->longLitTableOffset ||
+        r->smallWriteOffset || r->rolesWithStateCount || r->activeLeftCount || r->roseCount || r->rosePrefixCount ||
+        r->activeLeftIterOffset || r->eagerIterOffset || r->lastByteHistoryIterOffset || r->delayProgramOffset ||
+        r->anchoredProgramOffset || r->delay_count || r->anchored_count || r->handledKeyCount || r->lkeyCount ||
+        r->lopCount || r->ckeyCount || r->flushCombProgramOffset || r->lastFlushCombProgramOffset ||
+        br.reportEodOffset || br.reportZeroOffset || br.reportZeroEodOffset ||
+        (u64)r->nfaInfoOffset + (u64)n * sizeof(NfaInfo) > bcLen) {
+        return false;
+    }
+    const u8 *bc = (const u8 *)r;
+    std::vector<u32> eod;
+    for (u32 q = 0; q < n; q++) {
+        NfaInfo ni;
+        memcpy(&ni, bc + r->nfaInfoOffset + q * sizeof(NfaInfo), sizeof(ni));
+        if ((u64)ni.nfaOffset + sizeof(NFA) > bcLen) {
+            return false;
+        }
+        NFA nh;
+        memcpy(&nh, bc + ni.nfaOffset, sizeof(nh));
+        if (nh.flags & NFA_ACCEPTS_EOD) {
+            eod.push_back(q);
+        }
+    }
+    if (eod.empty() || !r->eodProgramOffset) {
+        return eod.empty() && !r->eodProgramOffset;
+    }
+    const u32 pc = r->eodProgramOffset;
+    const u32 endAt = pc + (u32)HSB_ROUNDUP(sizeof(InstrEnginesEod), INSTR_ALIGN);
+    if (!r->requiresEodCheck || pc % INSTR_ALIGN || (u64)endAt + sizeof(InstrEnd) > bcLen) {
+        return false;
+    }
+    InstrEnginesEod ee;
+    memcpy(&ee, bc + pc, sizeof(ee));
+    const std::vector<MmbitSparseIter> want = sparseIterator(eod, n);
+    const size_t iterBytes = want.size() * sizeof(MmbitSparseIter);
+    if (ee.code != OP_ENGINES_EOD || bc[endAt] != OP_END || (u64)ee.iter_offset + iterBytes > bcLen) {
+        return false;
+    }
+    for (size_t i = 0; i < want.size(); i++) {
+        MmbitSparseIter it;
+        memcpy(&it, bc + ee.iter_offset + i * sizeof(it), sizeof(it));
+        if (it.mask != want[i].mask || it.val != want[i].val) {
+            return false;
+        }
+    }
+    return true;
+}
+
 bool collectProgramReports(const u8 *bc, u32 bcLen, u32 prog, std::unordered_set<u32> *ex,
                            std::vector<ProgReport> *reports) {
     u32 pc = prog, furthest = prog;

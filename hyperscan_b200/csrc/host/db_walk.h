@@ -47,6 +47,11 @@ bool walkConfirm(const u8 *bc, u32 bcLen, u32 confOff, u32 nBuckets,
 /** Reports compiled with HS_FLAG_SINGLEMATCH in a pure-literal database. */
 hs_error_t collectExhaustible(const hs_database_t *db, std::unordered_set<u32> *ex);
 
+/** A FULL_ROSE database whose only contents are outfix engines (queues [0, queueCount), no matchers, roles,
+ * leftfixes, MPV, SOM, delays, boundary reports or logical combinations), with an EOD program that is absent or
+ * [ENGINES_EOD iter] END over exactly the queues whose engine accepts at EOD: what the device runs as it is. */
+bool outfixesOnly(const RoseEngine *r, u32 bcLen);
+
 /** Order records for delivery and apply the order-dependent report rules the
  * device skipped: one report per (block, id, to) (dedupe, src/report.h:55-119)
  * and, for HS_FLAG_SINGLEMATCH reports, only the first match per block

@@ -158,6 +158,196 @@ std::vector<u8> finishOutfixRose(Blob &blob, const std::vector<u8> &nfa, const R
     return out;
 }
 
+/* uncompressed state alignment of an engine in scratch (NFATraits<>::stateAlign, src/nfa/nfa_build_util.cpp:174-230:
+ * LimEx models max(alignof(state set), alignof(RepeatControl) = 8)) */
+u32 engineStateAlign(u8 type) {
+    switch (type) {
+    case NFA_MCCLELLAN_16: return 2;
+    case NFA_LIMEX_32: return 8;
+    case NFA_LIMEX_64:
+    case NFA_LIMEX_128: return 16;
+    case NFA_LIMEX_256: return 32;
+    case NFA_LIMEX_512: return 64;
+    default: return 1;
+    }
+}
+
+/* A database of several engines, each run as an outfix over the whole block, and nothing else: what the
+ * reference's back end emits for a set of outfixes without literals (ROSE_RUNTIME_FULL_ROSE; buildFinalEngine,
+ * src/rose/rose_build_bytecode.cpp:3609-3888).  hs_scan -> roseBlockExec (src/rose/block.c:345-422): every queue
+ * starts in blockInitSufPQ and runs to the end under catch-up; engines that accept at EOD are listed in the EOD
+ * program [ENGINES_EOD iter] END (makeEodProgram, :3334-3349; buildEodNfaIterator, :2276-2294). */
+std::vector<u8> finishEnginesRose(Blob &blob, const std::vector<std::vector<u8>> &engines, const RoseTail &t) {
+    const u32 n = (u32)engines.size();
+    std::vector<NfaInfo> infos(n);
+    memset(infos.data(), 0, sizeof(NfaInfo) * n);
+    std::vector<u32> eodQueues;
+    for (u32 q = 0; q < n; q++) {
+        std::vector<u8> eng = engines[q];
+        NFA hdr;
+        memcpy(&hdr, eng.data(), sizeof(hdr));
+        hdr.queueIndex = q; /* the engine knows its queue (buildOutfixes sets it) */
+        memcpy(eng.data(), &hdr, sizeof(hdr));
+        infos[q].nfaOffset = blob.add(eng.data(), eng.size(), 64);
+        if (hdr.flags & NFA_ACCEPTS_EOD) {
+            eodQueues.push_back(q);
+        }
+    }
+    RoseEngine r;
+    memset(&r, 0, sizeof(r));
+    r.runtimeImpl = RUNTIME_FULL_ROSE;
+    r.canExhaust = t.canExhaust ? 1 : 0;
+    r.mode = MODE_BLOCK;
+    r.ekeyCount = t.ekeyCount;
+    r.dkeyCount = t.dkeyCount;
+    r.dkeyLogSize = fatbitSize(r.dkeyCount);
+    r.invDkeyOffset = t.invDkeyOffset;
+    r.somLocationFatbitSize = fatbitSize(0);
+    r.activeArrayCount = n;
+    r.queueCount = n;
+    r.activeQueueArraySize = fatbitSize(n);
+    r.handledKeyFatbitSize = fatbitSize(0);
+    r.minWidth = t.minLen;
+    r.minWidthExcludingBoundaries = t.minLen;
+    r.maxBiAnchoredWidth = ROSE_BOUND_INF;
+    r.floatingDistance = ROSE_BOUND_INF;
+    r.delay_fatbit_size = fatbitSize(0);
+    r.anchored_fatbit_size = fatbitSize(0);
+    r.outfixBeginQueue = 0;
+    r.outfixEndQueue = n;
+    r.leftfixBeginQueue = n;
+    r.initMpvNfa = 0xffffffffu;
+    r.hasOutfixesInSmallBlock = 1; /* hasNonSmallBlockOutfix: none of them is in a small-block matcher */
+    if (!eodQueues.empty()) {
+        const std::vector<MmbitSparseIter> it = sparseIterator(eodQueues, n);
+        const u32 iterOffset = blob.add(it.data(), it.size() * sizeof(MmbitSparseIter), 8);
+        const u32 sz = instrSize<InstrEnginesEod>() + instrSize<InstrEnd>();
+        const u32 pc = blob.reserve(sz, INSTR_ALIGN);
+        InstrEnginesEod ee;
+        memset(&ee, 0, sizeof(ee));
+        ee.code = OP_ENGINES_EOD;
+        ee.iter_offset = iterOffset;
+        memcpy(blob.at(pc), &ee, sizeof(ee));
+        InstrEnd e;
+        e.code = OP_END;
+        memcpy(blob.at(pc + instrSize<InstrEnginesEod>()), &e, sizeof(e));
+        r.eodProgramOffset = pc;
+        r.requiresEodCheck = 1;
+    }
+    StateOffsets &so = r.stateOffsets;
+    u32 cur = 1; /* status byte; no roles */
+    so.activeLeafArray = cur;
+    so.activeLeafArray_size = mmbitSize(n);
+    cur += so.activeLeafArray_size;
+    so.activeLeftArray = so.longLitState = so.leftfixLagTable = so.anchorState = cur;
+    so.groups = cur;
+    so.groups_size = 0;
+    so.history = cur;
+    so.exhausted = cur;
+    so.exhausted_size = mmbitSize(r.ekeyCount);
+    cur += so.exhausted_size;
+    so.logicalVec = so.combVec = cur;
+    so.nfaStateBegin = cur;
+    /* allocateStateSpace (:2078-2099): stream state packed after rose's, full state in scratch, aligned */
+    u32 full = 0;
+    for (u32 q = 0; q < n; q++) {
+        NFA hdr;
+        memcpy(&hdr, engines[q].data(), sizeof(hdr));
+        infos[q].stateOffset = cur;
+        cur += hdr.streamStateSize;
+        full = HSB_ROUNDUP(full, engineStateAlign(hdr.type));
+        infos[q].fullStateOffset = full;
+        full += hdr.scratchStateSize;
+    }
+    so.end = cur;
+    r.stateSize = cur;
+    r.scratchStateSize = full;
+    r.nfaInfoOffset = blob.add(infos.data(), infos.size() * sizeof(NfaInfo), 4);
+    const u32 total = (u32)HSB_ROUNDUP(blob.base + blob.bytes.size(), 64);
+    r.size = total;
+    std::vector<u8> out(total, 0);
+    memcpy(out.data(), &r, sizeof(r));
+    memcpy(out.data() + blob.base, blob.bytes.data(), blob.bytes.size());
+    return out;
+}
+
+/* An expression of a set, with its report programs, and whether its own automaton determinises within 1 024 states */
+struct RegexMember {
+    const RegexPattern *p;
+    u32 report, reportBeforeNewline;
+    bool ownDfa;
+};
+
+/* The engines of a set whose expressions do not fit one automaton.  DFA groups first, since the DFA kernels scan
+ * several times faster than the wide LimEx models: in input order, a group takes the next expression while their
+ * union still determinises within 1 024 states.  The expressions whose own DFA is larger go to LimEx groups, each
+ * filled up to the 512-state model.  regexDfa = false: LimEx groups only. */
+std::vector<std::vector<u8>> partitionEngines(const std::vector<RegexMember> &members, bool regexDfa) {
+    std::vector<std::vector<u8>> engines;
+    auto add = [](RawNfa *nfa, const RegexMember &m) -> bool { /* false: the automaton would outgrow the model */
+        RawNfa trial = *nfa;
+        try {
+            regexNfaAdd(&trial, m.p->re.c_str(), m.p->flags, m.report, m.reportBeforeNewline, m.p->minLength);
+        } catch (const RegexError &) {
+            return false;
+        }
+        *nfa = std::move(trial);
+        return true;
+    };
+    std::vector<const RegexMember *> nfaOnly;
+    RawNfa group;
+    RawDfa groupDfa;
+    u32 count = 0;
+    auto closeDfa = [&]() {
+        if (count) {
+            minimizeDfa(&groupDfa);
+            engines.push_back(emitDfa(groupDfa, groupDfa.size() <= 256 ? DFA_MCCLELLAN8 : DFA_MCCLELLAN16, true));
+        }
+        regexNfaInit(&group);
+        count = 0;
+    };
+    regexNfaInit(&group);
+    for (const RegexMember &m : members) {
+        if (!regexDfa || !m.ownDfa) {
+            nfaOnly.push_back(&m);
+            continue;
+        }
+        RawNfa trial = group;
+        RawDfa d;
+        if (add(&trial, m) && determinize(trial, 1024, &d)) {
+            group = std::move(trial);
+            groupDfa = std::move(d);
+            count++;
+            continue;
+        }
+        closeDfa();
+        if (add(&group, m) && determinize(group, 1024, &groupDfa)) {
+            count = 1;
+        } else {
+            regexNfaInit(&group);
+            nfaOnly.push_back(&m);
+        }
+    }
+    closeDfa();
+    for (const RegexMember *m : nfaOnly) {
+        if (add(&group, *m)) {
+            count++;
+            continue;
+        }
+        engines.push_back(emitLimEx(group));
+        regexNfaInit(&group);
+        count = 0;
+        if (!add(&group, *m)) {
+            throw std::runtime_error("an expression outgrows the NFA model on its own");
+        }
+        count = 1;
+    }
+    if (count) {
+        engines.push_back(emitLimEx(group));
+    }
+    return engines;
+}
+
 /* Floating literal matcher + RoseEngine header around a finished program blob. */
 std::vector<u8> finishRose(Blob &blob, const std::vector<HwlmLit> &hl, const RoseTail &t,
                            const CompileOpts &opts, HwlmBuildInfo *info) {
@@ -226,6 +416,41 @@ std::vector<u8> finishRose(Blob &blob, const std::vector<HwlmLit> &hl, const Ros
 }
 
 } // namespace
+
+/* mmbBuildSparseIterator (src/util/multibit_build.cpp:156-190): one record per node of the multibit's 64-ary tree
+ * that holds a key, level by level, each level in key order.  A record's mask has the bits of its children; its val
+ * is where those children's records start, on the last level the count of keys before it. */
+std::vector<MmbitSparseIter> sparseIterator(const std::vector<u32> &keys, u32 totalBits) {
+    u32 ks = 0; /* mmbit_keyshift: 6 bits per level below the root */
+    for (u64 cap = 64; totalBits > 1 && cap < totalBits; cap <<= 6) {
+        ks += 6;
+    }
+    std::vector<MmbitSparseIter> out;
+    std::vector<size_t> levelStart;
+    for (u32 d = 0; d * 6 <= ks; d++) {
+        levelStart.push_back(out.size());
+        std::map<u32, u64> nodes; /* path above the level -> mask */
+        for (u32 k : keys) {
+            nodes[(u32)((u64)k >> (ks - 6 * d + 6))] |= 1ull << ((k >> (ks - 6 * d)) & 63);
+        }
+        for (const auto &n : nodes) {
+            MmbitSparseIter it;
+            memset(&it, 0, sizeof(it));
+            it.mask = n.second;
+            out.push_back(it);
+        }
+    }
+    levelStart.push_back(out.size());
+    for (size_t l = 0; l + 1 < levelStart.size(); l++) {
+        const bool last = l + 2 == levelStart.size();
+        u32 population = 0;
+        for (size_t i = levelStart[l]; i < levelStart[l + 1]; i++) {
+            out[i].val = (last ? 0 : (u32)levelStart[l + 1]) + population;
+            population += (u32)__builtin_popcountll(out[i].mask);
+        }
+    }
+    return out;
+}
 
 std::vector<u8> buildLiteralRose(const std::vector<LitPattern> &patsIn,
                                  const CompileOpts &opts, HwlmBuildInfo *info) {
@@ -753,6 +978,8 @@ std::vector<u8> buildRegexRose(const std::vector<RegexPattern> &pats, const Comp
         progOf[key] = prog;
         return prog;
     };
+    std::vector<RegexMember> members;
+    bool overflow = false; /* the set's positions exceed one automaton: it is split into several engines */
     for (const RegexPattern &p : pats) {
         try {
             const RegexInfo ri = regexInfo(p.re.c_str(), p.flags);
@@ -783,6 +1010,7 @@ std::vector<u8> buildRegexRose(const std::vector<RegexPattern> &pats, const Comp
                                        "expression.", (int)p.index};
                 }
             }
+            bool ownDfa = false;
             {
                 /* "Pattern can never match." (can_never_match after resolveAsserts, src/nfagraph/ng.cpp:330-350): the
                  * expression's own automaton, determinised and minimised, is the dead state alone */
@@ -790,7 +1018,8 @@ std::vector<u8> buildRegexRose(const std::vector<RegexPattern> &pats, const Comp
                 regexNfaInit(&own);
                 regexNfaAdd(&own, p.re.c_str(), p.flags, 1, ri.needsAdjust ? 2 : 0, p.minLength);
                 RawDfa d;
-                if (determinize(own, 1024, &d)) {
+                ownDfa = determinize(own, 1024, &d);
+                if (ownDfa) {
                     minimizeDfa(&d);
                     if (d.size() < 2) {
                         throw CompileError{"Pattern can never match.", (int)p.index};
@@ -798,7 +1027,15 @@ std::vector<u8> buildRegexRose(const std::vector<RegexPattern> &pats, const Comp
                 }
             }
             minLen = std::min<u32>(minLen, (u32)std::max<u64>(ri.minLen, std::min<u64>(p.minLength, 0xffffffffu)));
-            regexNfaAdd(&nfa, p.re.c_str(), p.flags, program(p, 0), ri.needsAdjust ? program(p, -1) : 0, p.minLength);
+            if (!overflow) {
+                try {
+                    regexNfaAdd(&nfa, p.re.c_str(), p.flags, program(p, 0), ri.needsAdjust ? program(p, -1) : 0, p.minLength);
+                } catch (const RegexError &) {
+                    overflow = true; /* the expression alone fits (its own automaton was built above): the set does not */
+                }
+            }
+            const u32 report = program(p, 0); /* (made above while the set fits: the same programs) */
+            members.push_back({&p, report, ri.needsAdjust ? program(p, -1) : 0, ownDfa});
         } catch (const RegexError &e) {
             throw CompileError{e.msg, (int)p.index};
         }
@@ -814,6 +1051,15 @@ std::vector<u8> buildRegexRose(const std::vector<RegexPattern> &pats, const Comp
     }
     t.invDkeyOffset = blob.add(inv.data(), inv.size() * sizeof(u32), 4);
     t.canExhaust = allHighlander;
+    if (overflow) {
+        std::vector<std::vector<u8>> engines;
+        try {
+            engines = partitionEngines(members, opts.regexDfa);
+        } catch (const std::runtime_error &e) {
+            throw CompileError{std::string("Unable to build the NFA: ") + e.what(), -1};
+        }
+        return finishEnginesRose(blob, engines, t);
+    }
     std::vector<u8> eng;
     try {
         /* small automata run as DFAs, as in the reference (ng_mcclellan before LimEx); the report programs are

@@ -55,8 +55,10 @@ static const size_t LIMIT_LITERAL_COUNT = 8000000;
 std::vector<u8> buildLiteralRose(const std::vector<LitPattern> &pats,
                                  const CompileOpts &opts, HwlmBuildInfo *info);
 
-/** Expressions that need an NFA (regex_nfa.h): ONE LimEx-32 engine over all of them, run as the
- * database's single outfix (ROSE_RUNTIME_SINGLE_OUTFIX).  Block mode only.  Throws CompileError. */
+/** Expressions that need an NFA (regex_nfa.h): ONE engine over all of them (McClellan-8 / -16 when the automaton
+ * determinises small enough, else LimEx), run as the database's single outfix (ROSE_RUNTIME_SINGLE_OUTFIX).  A set
+ * whose positions do not fit one 512-state automaton is split into several engines, each an outfix of a
+ * FULL_ROSE database that holds nothing else.  Block mode only.  Throws CompileError. */
 struct RegexPattern {
     std::string re;
     unsigned flags = 0;
@@ -66,6 +68,10 @@ struct RegexPattern {
     u64 minLength = 0;                    /* hs_expr_ext: shortest match that counts (regex_nfa.cpp) */
 };
 std::vector<u8> buildRegexRose(const std::vector<RegexPattern> &pats, const CompileOpts &opts);
+
+/** The sparse iterator over `keys` of a multibit of totalBits bits, as the reference lays it out
+ * (mmbBuildSparseIterator): what an ENGINES_EOD instruction walks. */
+std::vector<MmbitSparseIter> sparseIterator(const std::vector<u32> &keys, u32 totalBits);
 
 /** Test hook: pure-literal block database from raw literal programs (`area`
  * is placed at programAreaBase(); lits[i].id = its program's offset in area). */

@@ -321,6 +321,7 @@ enum RoseOp {
     OP_DEDUPE_AND_REPORT = 37,
     OP_FINAL_REPORT = 38,
     OP_CHECK_EXHAUSTED = 39,
+    OP_ENGINES_EOD = 48,
     OP_SQUASH_GROUPS = 43,
     OP_CHECK_LONG_LIT = 51,
     OP_CHECK_LONG_LIT_NOCASE = 52,
@@ -354,6 +355,10 @@ struct InstrSquashGroups { u8 code; u64 groups; };
 struct InstrCheckLit { u8 code; u32 lit_offset; u32 lit_length; u32 fail_jump; }; /* MED + LONG */
 struct InstrIncludedJump { u8 code, squash; u32 child_offset; };
 struct InstrSetExhaust { u8 code; u32 ekey; };
+struct InstrEnginesEod { u8 code; u32 iter_offset; }; /* the queues of a sparse iterator at EOD */
+
+/* one record of a sparse multibit iterator (src/util/multibit_internal.h:59-62) */
+struct MmbitSparseIter { u64 mask; u32 val; };
 
 /* ---- NFA engines (DFA subset): src/nfa/nfa_internal.h:53-126,
  *      src/nfa/mcclellan_internal.h:36-106 -------------------------------- */
